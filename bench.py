@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- PAN control steps/sec on the BASELINE.json north-star workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload C4] [--dump-outputs DIR]
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" = one batched PAN.forward (iter_num fixed at the config's K by iter_threshold = 0) over
@@ -15,6 +15,10 @@ all_gather, inside the timed region).  Prints ONE JSON line (rank 0).
   cpu_baseline the CPU oracle (port of the reference path) on the box's host cores, bounded sample
 
 --impl reference times that CPU path alone, on all host cores (rank 0 only).
+
+--dump-outputs DIR (C1 ... C5, --impl ours) writes what the last timed step returned -- the trajectories S, U, D and
+min_distance of every environment, unpacked from ShardedPAN.step -- as float32 DIR/<name>.npy, so that two builds run with
+the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -33,6 +37,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np  # noqa: E402
 
 METRIC = "PAN control steps/sec (batched envs, T x N x K)"
+DUMP_LIMIT_BYTES = 64 << 20
 UNIT = "env-steps/s"
 F_PT = 8576  # GEMM FLOPs per point-step at E=4: 2*(2*32 + 4*32*32 + 32*4)   (SURVEY.md 8d)
 
@@ -284,7 +289,7 @@ class PanBench:
         for i in range(steps):
             self.flush.zero_()  # L2 flush, outside the per-step events
             ev[i][0].record()
-            self.step(i)
+            self.last_out = self.step(i)
             ev[i][1].record()
         self.barrier()
         launches = (self.lib.nb_launch_count() - l0) // max(1, steps)
@@ -310,6 +315,23 @@ class PanBench:
 
     def close(self):
         self.pan.close()
+
+
+def dump_outputs(dirname, packed, T):
+    """S, U, D, min_distance of one step (the packed (envs, 64) result of ShardedPAN.step) as float32 .npy files; above
+    DUMP_LIMIT_BYTES a fixed seeded sample of environments, whose indices go to env_index.npy."""
+    from neupan_b200.parallel import unpack_results
+
+    os.makedirs(dirname, exist_ok=True)
+    packed = packed.float().cpu()
+    n = packed.shape[0]
+    keep = DUMP_LIMIT_BYTES // (4 * packed.shape[1] + 8)
+    if n > keep:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        packed = packed[idx]
+        np.save(os.path.join(dirname, "env_index.npy"), idx.astype(np.float64))
+    for name, a in zip(("S", "U", "D", "min_distance"), unpack_results(packed, T)):
+        np.save(os.path.join(dirname, f"{name}.npy"), np.ascontiguousarray(a.numpy(), np.float32))
 
 
 def run_ours(args):
@@ -345,7 +367,9 @@ def run_ours(args):
     clocks = sampler.stop() if rank == 0 else None
     status_bad = int((hb.pan.status != 0).sum().item())
     iters_mean = float(hb.pan.iterations.float().mean().item())
-    e2e_ms = hb.time_e2e(max(2, min(args.steps, 5)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, hb.last_out, T)
+    e2e_ms = hb.time_e2e(args.steps)
     h2d, d2h = hb.bytes_per_step()
     pan, flush, dsets = hb.pan, hb.flush, hb.dsets
 
@@ -774,7 +798,7 @@ def run_train(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="C4")
@@ -785,7 +809,12 @@ def main():
     ap.add_argument("--iter-threshold", type=float, default=0.0, help="PAN stop criterion (pan.py:243); 0 forces exactly K iterations (the headline), the reference default is 0.1")
     ap.add_argument("--nrmp-warm", type=int, default=0, help="NB_OPT_NRMP_WARM: 1 = NRMP solves of PAN iterations k > 0 start from iteration k-1's solution")
     ap.add_argument("--overlap", type=int, default=2, help="env sub-batches pipelined on internal streams (NB_OPT_OVERLAP)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (PAN workloads C1 ... C5, --impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload in ("train", "control", "ipath", "scan")):
+        ap.error("--dump-outputs is implemented for the PAN workloads (C1 ... C5) with --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload == "train":
         run_train(args)

@@ -1,13 +1,12 @@
 """Pins oracle/dune.py (the CPU restatement of the DUNE half) against the reference's own code:
-golden vectors produced by that code (tests/golden/ref_dune_*.npz, made by make_golden.py) and,
-when /root/reference is present, the live import."""
+golden vectors produced by that code (tests/golden/ref_dune_*.npz, made by make_golden.py, and
+tests/golden/ref_calls.npz, made by make_golden_refcalls.py)."""
 import numpy as np
 import pytest
 import torch
 
 from helpers import GOLDEN, weights_path
 from oracle import dune as od
-from oracle.refload import reference_available
 
 
 @pytest.mark.parametrize("model", ["diff", "acker", "polygon"])
@@ -36,32 +35,21 @@ def test_dune_matches_reference_golden(model, case):
         assert torch.equal(d_ref, d_stb)
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present on this machine")
 def test_dune_matches_live_reference():
-    import types
+    """The reference's DUNE.forward on its acker checkpoint (recorded in ref_calls.npz) vs the oracle on the weights fixture."""
+    import hashlib
 
-    from oracle.refload import REFERENCE_ROOT, load_reference
-
-    load_reference()
-    from neupan.blocks import DUNE, PAN
-    from neupan.robot import robot as RefRobot
-
-    rr = RefRobot(10, 0.1, kinematics="acker", length=4.6, width=1.6, wheelbase=3)
-    ck = f"{REFERENCE_ROOT}/example/model/acker_robot_default/model_5000.pth"
-    dune = DUNE(10, ck, rr, 80, {})
-    fake = types.SimpleNamespace(T=10, dt=0.1, dune_max_num=80, printed=True, print_once=lambda *_: None)
-    fake.point_state_transform = types.MethodType(PAN.point_state_transform, fake)
-    g = torch.Generator().manual_seed(3)
-    nom_s = torch.randn(3, 11, generator=g); pts = 6 * torch.randn(2, 200, generator=g); vel = torch.randn(2, 200, generator=g)
-    pf, Rl, pl = PAN.generate_point_flow(fake, nom_s, pts, vel)
-    mu_r, lam_r, sp_r = dune(pf, Rl, pl)
-    w = od.load_weights(ck)
+    z = np.load(f"{GOLDEN}/ref_calls.npz")
+    nom_s, pts, vel = (torch.from_numpy(z[f"dune.{k}"]) for k in ("nom_s", "points", "velocities"))
+    w = od.load_weights(weights_path("acker"))
     p0, R, pl2 = od.point_flow(nom_s, pts, vel, 10, 0.1, 80)
-    mu, lam, sp, md, _ = od.dune_forward(w, torch.from_numpy(rr.G).float(), torch.from_numpy(rr.h).float(), p0, R, pl2, stable=False)
-    assert all(torch.equal(a, b) for a, b in zip(mu, mu_r))
-    assert all(torch.equal(a, b) for a, b in zip(lam, lam_r))
-    assert all(torch.equal(a, b) for a, b in zip(sp, sp_r))
-    assert float(md) == float(dune.min_distance)
+    mu, lam, sp, md, _ = od.dune_forward(w, torch.from_numpy(z["dune.G"]), torch.from_numpy(z["dune.h"]), p0, R, pl2, stable=False)
+    assert np.array_equal(torch.stack(mu).numpy(), z["dune.mu"])
+    assert np.array_equal(torch.stack(lam).numpy(), z["dune.lam"])
+    assert np.array_equal(torch.stack(sp).numpy(), z["dune.sorted_points"])
+    assert np.float32(md) == z["dune.min_distance"]
     # weights fixture == checkpoint
-    wz = od.load_weights(weights_path("acker"))
-    assert all(torch.equal(w[k], wz[k]) for k in w)
+    h = hashlib.sha256()
+    for k in sorted(w):
+        h.update(k.encode()); h.update(np.ascontiguousarray(w[k].numpy(), np.float32).tobytes())
+    assert h.hexdigest() == str(z["dune.checkpoint_sha256"])

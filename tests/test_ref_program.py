@@ -1,72 +1,50 @@
 """Pins the NRMP convex program to the REFERENCE'S OWN CODE (VERDICT r1, weak #1 / next #2).
 
 ``oracle/cvx_shim.py`` stands in for cvxpy / cvxpylayers, so ``neupan/blocks/nrmp.py:263-383`` and
-``neupan/robot/robot.py:73-236`` execute unmodified and produce the program as arrays.  Checked here, for
+``neupan/robot/robot.py:73-236`` execute unmodified and produce the program as arrays; ``tests/golden/ref_calls.npz``
+holds those arrays and what the reference returned (made by ``tests/golden/make_golden_refcalls.py``).  Checked here, for
 diff / acker / omni, scalar and vector q_s, with and without obstacle rows:
 
 * the reference's objective equals ``oracle.nrmp.objective`` at random points (feasible or not);
 * the oracle's optimum (float64 interior point, ``oracle/ipm.py``) satisfies the reference's constraints and passes a
   solver-free KKT certificate *of the reference's program*;
-* the reference's own ``NRMP.forward`` (shim solver: HiGHS + active-set polish) returns the same trajectory;
+* the reference's own ``NRMP.forward`` (shim solver: HiGHS + active-set polish) returned the same trajectory;
 * the reference's whole ``PAN.forward`` (its torch DUNE code + its NRMP through the shim) agrees with ``oracle.pan.OraclePAN``.
 
-Needs /root/reference (skipped on the GPU box).  What stays unobservable: ECOS' own output.
+What stays unobservable: ECOS' own output.
 """
+import importlib.util
+import os
+
 import numpy as np
 import pytest
-import torch
 
-from helpers import CONFIGS, make_inputs, oracle_factory, robot_spec, weights_path
-from oracle import dune as od, ipm as oipm, nrmp as onr, refload
+from helpers import GOLDEN, CONFIGS, make_inputs, oracle_factory, robot_spec
+from oracle import dune as od, ipm as oipm, nrmp as onr
 
-pytestmark = pytest.mark.skipif(not refload.reference_available(), reason="needs /root/reference")
-
-CASES = [("C1", {}, None), ("C2", {}, None), ("C4", {}, None), ("C5", {}, None),
-         ("C4", dict(q_s=[0.5, 1.5, 0.25]), None), ("C2", dict(q_s=[1.0, 0.3, 2.0], p_u=0.7, eta=8.0, d_max=1.5, d_min=0.2), None),
-         ("C1", {}, 0), ("C5", dict(q_s=[1.0, 2.0, 3.0]), 0)]
-
-
-def _ref_layer(cfg, adjust, M):
-    refload.load_reference()
-    from neupan.blocks.nrmp import NRMP
-    from neupan.robot import robot as RefRobot
-
-    rb = RefRobot(cfg.T, cfg.dt, **cfg.robot_kwargs)
-    return NRMP(cfg.T, cfg.dt, rb, nrmp_max_num=cfg.M if M is None else M, **adjust), rb
-
-
-def _dune_lists(cfg, inp, b=0):
-    """mu / lam / sorted point lists of one environment from the (reference-pinned) DUNE oracle."""
-    rb, spec = robot_spec(cfg)
-    w = od.load_weights(weights_path(cfg.model))
-    G, h = torch.from_numpy(spec.G).float(), torch.from_numpy(spec.h.reshape(-1, 1)).float()
-    t = lambda a: None if a is None else torch.from_numpy(a[b])
-    vel = None if inp["velocities"] is None else t(inp["velocities"])
-    p0, R, p = od.point_flow(t(inp["nom_s"]), t(inp["points"]), vel, cfg.T, cfg.dt, cfg.N)
-    mu, lam, sp, _, _ = od.dune_forward(w, G, h, p0, R, p)
-    return mu, lam, sp, h, spec
+_spec = importlib.util.spec_from_file_location("make_golden_refcalls", os.path.join(GOLDEN, "make_golden_refcalls.py"))
+mgr = importlib.util.module_from_spec(_spec)
+_spec.loader.exec_module(mgr)
+GOLD = np.load(os.path.join(GOLDEN, "ref_calls.npz"))
+CASES = mgr.CASES
 
 
 def _problem_and_reference(cname, adjust_over, M, scene="obstacles", env=0):
-    cfg = CONFIGS[cname]
-    adjust = dict(cfg.adjust); adjust.update(adjust_over)
-    Mv = cfg.M if M is None else M
-    inp = make_inputs(cfg, B=1, N=min(cfg.N, 120), scene=scene, env_offset=env)
-    layer, _ = _ref_layer(cfg, adjust, M)
-    t = lambda a: torch.from_numpy(a[0])
-    nom_s, nom_u, ref_s, ref_us = t(inp["nom_s"]), t(inp["nom_u"]), t(inp["ref_s"]), t(inp["ref_us"])
+    """(cfg, the reference's program, the oracle's program, the reference's float64 solution, its (S, U, D)) of a case."""
+    cfg, adjust, Mv, inp = mgr.program_inputs(cname, adjust_over, M, scene, env)
+    i = CASES.index((cname, adjust_over, M))
+    can = mgr.canonical_from(GOLD, f"program.{i}")
     if Mv > 0:
-        mu, lam, sp, h, spec = _dune_lists(cfg, inp)
+        mu, lam, sp, h, spec = mgr.dune_lists(cfg, inp)
         fa, fb = od.nrmp_coefficients(h, mu, lam, sp, cfg.T, Mv)
         fa, fb = fa.numpy(), fb.numpy()
-        S, U, D = layer.forward(nom_s, nom_u, ref_s, ref_us, mu, lam, sp)
     else:
         _, spec = robot_spec(cfg)
         fa = fb = None
-        S, U, D = layer.forward(nom_s, nom_u, ref_s, ref_us)
     adj = onr.Adjust(**adjust)
-    prob = onr.build_problem(spec, adj, nom_s.numpy(), nom_u.numpy(), ref_s.numpy(), ref_us.numpy(), fa, fb, Mv)
-    return cfg, layer, prob, (S, U, D)
+    prob = onr.build_problem(spec, adj, inp["nom_s"][0], inp["nom_u"][0], inp["ref_s"][0], inp["ref_us"][0], fa, fb, Mv)
+    ref = (GOLD[f"program.{i}.S"], GOLD[f"program.{i}.U"], GOLD[f"program.{i}.D"] if Mv > 0 else None)
+    return cfg, can, prob, GOLD[f"program.{i}.x"], ref
 
 
 def _stack_x(prob, S, U, D):
@@ -78,8 +56,7 @@ def _stack_x(prob, S, U, D):
 
 @pytest.mark.parametrize("cname,adjust,M", CASES)
 def test_reference_objective_equals_oracle_objective(cname, adjust, M):
-    cfg, layer, prob, _ = _problem_and_reference(cname, adjust, M)
-    can = layer.nrmp_layer.last_canonical
+    cfg, can, prob, _, _ = _problem_and_reference(cname, adjust, M)
     rng = np.random.default_rng(5)
     for _ in range(6):
         S = prob.nom_s + rng.normal(0, 0.5, prob.nom_s.shape)
@@ -91,65 +68,49 @@ def test_reference_objective_equals_oracle_objective(cname, adjust, M):
 
 @pytest.mark.parametrize("cname,adjust,M", CASES)
 def test_oracle_optimum_is_optimal_for_the_reference_program(cname, adjust, M):
-    cfg, layer, prob, (Sr, Ur, Dr) = _problem_and_reference(cname, adjust, M)
-    can = layer.nrmp_layer.last_canonical
+    cfg, can, prob, xr, (Sr, Ur, Dr) = _problem_and_reference(cname, adjust, M)
     S, U, D, _ = oipm.solve_ipm(prob)
     x = _stack_x(prob, S, U, D)
     res, viol = can.kkt_certificate(x, act_tol=1e-7)
     scale = max(1.0, float(np.abs(can.gradient(x)).max()))
     assert viol < 1e-8, viol  # the reference's constraints hold at the oracle's optimum
     assert res < 2e-6 * scale, (res, scale)  # and its gradient is a combination of active normals
-    # the reference's own forward (shim solver) lands on the same point
-    xr = layer.nrmp_layer.last_x  # float64, before the reference's cast to float32 (nrmp.py:145-148)
+    # the reference's own forward (shim solver) lands on the same point; xr: float64, before its cast to float32 (nrmp.py:145-148)
     assert can.violation(xr) < 1e-8
     assert can.objective(x) <= can.objective(xr) + 1e-8 * max(1.0, abs(can.objective(xr)))
-    assert np.abs(U - Ur.numpy()).max() < 2e-5 and np.abs(S - Sr.numpy()).max() < 2e-5
+    assert np.abs(U - Ur).max() < 2e-5 and np.abs(S - Sr).max() < 2e-5
     if prob.M > 0:
-        assert np.abs(D - Dr.numpy()).max() < 2e-5
+        assert np.abs(D - Dr).max() < 2e-5
 
 
 def test_reference_parameter_values_equal_oracle_parameters():
     """generate_parameter_value of the reference (nrmp.py:152-166, robot.py:239-316) vs oracle.nrmp.build_problem: bit for bit."""
-    for cname in ("C1", "C2", "C5"):
-        cfg, layer, prob, _ = _problem_and_reference(cname, {}, None)
-        inp = make_inputs(cfg, B=1, N=min(cfg.N, 120), scene="obstacles")
-        t = lambda a: torch.from_numpy(a[0])
-        mu, lam, sp, h, spec = _dune_lists(cfg, inp)
-        vals = layer.generate_parameter_value(t(inp["nom_s"]), t(inp["nom_u"]), t(inp["ref_s"]), t(inp["ref_us"]), mu, lam, sp)
+    for cname in mgr.PARAM_CONFIGS:
+        cfg, _, prob, _, _ = _problem_and_reference(cname, {}, None)
+        vals = [GOLD[f"params.{cname}.{k}"] for k in range(int(GOLD[f"params.{cname}"]))]
         T = cfg.T
-        assert np.array_equal(vals[0].numpy(), prob.nom_s.astype(np.float32))
-        assert np.array_equal(vals[1].detach().numpy(), prob.gamma_a.astype(np.float32))
-        assert np.array_equal(vals[2].detach().numpy(), prob.gamma_b.astype(np.float32))
+        assert np.array_equal(vals[0], prob.nom_s.astype(np.float32))
+        assert np.array_equal(vals[1], prob.gamma_a.astype(np.float32))
+        assert np.array_equal(vals[2], prob.gamma_b.astype(np.float32))
         for k in range(T):
-            assert np.array_equal(vals[3 + k].numpy(), prob.A[k].astype(np.float32))
-            assert np.array_equal(vals[3 + T + k].numpy(), prob.B[k].astype(np.float32))
-            assert np.array_equal(vals[3 + 2 * T + k].numpy().reshape(-1), prob.C[k].astype(np.float32))
-            assert np.array_equal(vals[3 + 3 * T + k].numpy(), prob.fa[k].astype(np.float32))
-            assert np.array_equal(vals[3 + 4 * T + k].numpy().reshape(-1), prob.fb[k].astype(np.float32))
+            assert np.array_equal(vals[3 + k], prob.A[k].astype(np.float32))
+            assert np.array_equal(vals[3 + T + k], prob.B[k].astype(np.float32))
+            assert np.array_equal(vals[3 + 2 * T + k].reshape(-1), prob.C[k].astype(np.float32))
+            assert np.array_equal(vals[3 + 3 * T + k], prob.fa[k].astype(np.float32))
+            assert np.array_equal(vals[3 + 4 * T + k].reshape(-1), prob.fb[k].astype(np.float32))
 
 
 @pytest.mark.parametrize("cname,K", [("C1", 2), ("C2", 3), ("C5", 2)])
 def test_reference_pan_forward_equals_oracle_pan(cname, K):
     """The reference's PAN.forward end to end (pan.py:109-147) with only the solver swapped vs OraclePAN."""
-    refload.load_reference()
-    from neupan.blocks.pan import PAN as RefPAN
-    from neupan.robot import robot as RefRobot
-
     cfg = CONFIGS[cname]
     N = min(cfg.N, 150)
     inp = make_inputs(cfg, B=2, N=N, scene="obstacles")
-    import tempfile, os
-    w = od.load_weights(weights_path(cfg.model))
-    with tempfile.TemporaryDirectory() as tmp:
-        ck = os.path.join(tmp, "model.pth")
-        torch.save({k: v for k, v in w.items()}, ck)
-        for b in range(2):
-            rb = RefRobot(cfg.T, cfg.dt, **cfg.robot_kwargs)
-            rp = RefPAN(cfg.T, cfg.dt, rb, iter_num=K, dune_max_num=N, nrmp_max_num=cfg.M, dune_checkpoint=ck, iter_threshold=0.0, adjust_kwargs=dict(cfg.adjust))
-            t = lambda a: None if a is None else torch.from_numpy(a[b])
-            S, U, D = rp(t(inp["nom_s"]), t(inp["nom_u"]), t(inp["ref_s"]), t(inp["ref_us"]), t(inp["points"]), t(inp["velocities"]))
-            op_ = oracle_factory(cfg, K=K, N=N)()
-            vel = None if inp["velocities"] is None else inp["velocities"][b]
-            So, Uo, Do = op_.forward(inp["nom_s"][b], inp["nom_u"][b], inp["ref_s"][b], inp["ref_us"][b], inp["points"][b], vel)
-            assert np.abs(S.numpy() - So).max() < 1e-4 and np.abs(U.numpy() - Uo).max() < 1e-4 and np.abs(D.numpy() - Do).max() < 1e-4
-            assert abs(float(rp.min_distance) - op_.min_distance) < 1e-6
+    for b in range(2):
+        g = f"pan.{cname}.{K}.{b}"
+        S, U, D = GOLD[f"{g}.S"], GOLD[f"{g}.U"], GOLD[f"{g}.D"]
+        op_ = oracle_factory(cfg, K=K, N=N)()
+        vel = None if inp["velocities"] is None else inp["velocities"][b]
+        So, Uo, Do = op_.forward(inp["nom_s"][b], inp["nom_u"][b], inp["ref_s"][b], inp["ref_us"][b], inp["points"][b], vel)
+        assert np.abs(S - So).max() < 1e-4 and np.abs(U - Uo).max() < 1e-4 and np.abs(D - Do).max() < 1e-4
+        assert abs(float(GOLD[f"{g}.min_distance"]) - op_.min_distance) < 1e-6

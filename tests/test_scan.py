@@ -5,7 +5,7 @@ import os
 import numpy as np
 import pytest
 
-from oracle import refload, scan as oscan
+from oracle import scan as oscan
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 _spec = importlib.util.spec_from_file_location("make_golden_scan", os.path.join(HERE, "golden", "make_golden_scan.py"))
@@ -32,13 +32,22 @@ def test_oracle_reproduces_reference_golden_vectors(name):
         assert np.array_equal(vel, g["vel_out"])
 
 
-@pytest.mark.skipif(not refload.reference_available(), reason="/root/reference not mounted")
 def test_golden_vectors_are_current():
-    """Regenerating from the reference in this container gives the committed fixture."""
-    ref = refload.load_reference().neupan
+    """The reference's scan_to_point_velocity, replayed from its recorded calls (ref_calls.npz) on the fixture's inputs, packed
+    by oracle.scan.scan_batch, gives the committed fixture."""
+    calls = np.load(os.path.join(HERE, "golden", "ref_calls.npz"))
     (B, R, scan, off, ar, ds, mp, vm), g = _case("velocity_stride")
-    fn_v = lambda st, sc, o, a, d: ref.scan_to_point_velocity(None, st, sc, o, a, d)
+    seen = []
+
+    def fn_v(st, sc, o, a, d):
+        i = len(seen)
+        seen.append(i)
+        assert np.array_equal(st, calls[f"scan.{i}.state"]) and np.array_equal(sc["ranges"], calls[f"scan.{i}.ranges"])
+        assert np.array_equal(sc["velocity"], calls[f"scan.{i}.velocity"])
+        return calls[f"scan.{i}.points"], calls[f"scan.{i}.vel"]
+
     pts, vel, cnt = oscan.scan_batch(g["states"], g["ranges"], scan, off, ar, ds, mp, g["velocity"], True, fn_velocity=fn_v)
+    assert len(seen) == int(calls["scan.calls"])
     assert np.array_equal(pts, g["points"]) and np.array_equal(vel, g["vel_out"]) and np.array_equal(cnt, g["counts"])
 
 
