@@ -42,14 +42,17 @@ struct DuneParams {
   unsigned* screen_stats;   // [0] max |d~ - d| / sum|t| over candidates (float bits), [1] items sent to the exact kernel, [2] candidates, [3] items screened
   float c_mu;               // bound on |mu~_e - mu_e| of the screening network
   int32_t* flag_list;       // (B (T+1)) the items with cand_cnt == -1, in the order the screen kernel met them
-  int32_t* flag_count;      // (3) [0] their number, [1] / [2] the lengths of the two refine lists; zeroed by the launcher before the screen kernel
+  int32_t* flag_count;      // (4) [0] their number, [1] / [2] the lengths of the two refine lists, [3] the item counter of dune_screen_warp_kernel;
+                            // zeroed by the launcher before the screen kernel
   int32_t* refine_list;     // (2 B (T+1)) work lists of dune_refine_kernel, appended by the screen kernels: [0, B (T+1)) the items with 1..16
                             // candidates (two of them share a warp), [B (T+1), 2 B (T+1)) those with 17..32 (one warp each)
   int only_flagged;         // exact kernel: process only the items of flag_list
   int skip_t0;              // screen kernels: step-0 items are skipped (cand_cnt = 0) and keep the outputs of the previous launch -- set by
                             // nb_pan_forward for PAN iterations k > 0: nom_s[:, 0] is the fixed initial state (robot.py:234; the NRMP kernel
                             // copies the column bit for bit), so item (b, 0) has the same inputs and the same result in every iteration
-  int screen_mma;           // launcher hint (NB_OPT_DUNE_SCREEN_MMA): 1 = screening pass on mma.sync (dune_screen_mma_kernel.cuh) where N <= 512
+  int screen_mma;           // launcher hint (NB_OPT_DUNE_SCREEN_MMA): screening pass on mma.sync (dune_screen_mma_kernel.cuh) where N <= 1024,
+                            // 1 = one warp per item (dune_screen_warp_kernel) if the launch has an item per resident warp, else one CTA per
+                            // item (dune_screen_mma_kernel); 2 / 3 = always the CTA / warp shape; 0 = tcgen05
   int calibrate;            // screen kernel: items with N <= 32 are NOT short-cut: all their points become candidates with their screened
                             // distance, so that the refine kernel's statistics compare the two networks on every point (nb_pan calibration)
 };

@@ -12,7 +12,9 @@
 // points (585 clk of the legacy tensor pipe per scheduler) against 792 clk of MUFU.TANH -- the exact path (3 passes, 204 HMMA)
 // is the one that needs tcgen05, and keeps it (dune_refine_kernel / dune_tcp_kernel).
 //
-// Mapping (clouds of up to 1024 points; see the kP template parameter): CTA = 4 warps = one (environment, step) item at a time; pass p, warp w: points [128 p + 32 w, +32) as two m16 tiles.
+// Two shapes share the per-tile code below (sm::screen_point): dune_screen_warp_kernel (the default, one warp per (environment, step)
+// item, at the end of this file) and dune_screen_mma_kernel (one CTA of 4 warps per item, kept for A/B timing: NB_SCREEN_MMA=2).
+// Mapping of dune_screen_mma_kernel (clouds of up to 1024 points; see the kP template parameter): CTA = 4 warps = one item at a time; pass p, warp w: points [128 p + 32 w, +32) as two m16 tiles.
 // Lane (g = lane >> 2, tq = lane & 3) holds rows g, g+8 (tile 0), g, g+8 (tile 1) -- "row slots" 0..3 = local points g + 8 r --
 // and columns 8 j + 2 tq, +1 (j = 0..3) of every 32-wide activation; it OWNS local point 8 tq + g (coordinates in, key out), so
 // the four row slots of a quad are exactly the points its four lanes own (one shuffle each way, no shared memory).
@@ -154,6 +156,107 @@ __device__ __forceinline__ void dense_frag(const uint4* __restrict__ wl, const f
     }
 }
 
+// the screen image of dune_screen_kernel (K-major UMMA layout, hi halves) re-ordered into mma.sync B fragments, the permuted fp32
+// vectors and the bias fragments, by the 128 threads of a CTA
+__device__ __forceinline__ void stage_operands(const unsigned char* __restrict__ image, unsigned char* smem_dyn, int tid) {
+  using I = TcImage;
+  uint4* wfrag = reinterpret_cast<uint4*>(smem_dyn);
+  float* vec = reinterpret_cast<float*>(smem_dyn + kFragBytes);
+  float4* biasq = reinterpret_cast<float4*>(smem_dyn + kFragBytes + kVecBytes);
+  uint32_t* wf = reinterpret_cast<uint32_t*>(wfrag);
+  for (int x = tid; x < kFragBytes / 4; x += 128) {
+    const int c = x & 3, ln = (x >> 2) & 31, jp = (x >> 7) & 1, s = (x >> 8) & 1, l = x >> 9;
+    const int n = 8 * (2 * jp + (c >> 1)) + (ln >> 2), k = 16 * s + 2 * (ln & 3) + 8 * (c & 1);
+    const size_t off = (size_t)l * I::kLayerStride + (size_t)(k / 16) * 1024 + ((k % 16) / 8) * 512 + (n / 8) * 128 + (n % 8) * 16 + (k % 8) * 2;
+    wf[x] = *reinterpret_cast<const uint32_t*>(image + off);
+  }
+  const float* fl = reinterpret_cast<const float*>(image + I::kFloatOff);
+  for (int x = tid; x < kVecs * 32; x += 128) {
+    const int v = x >> 5, e = x & 31, q = e >> 3, j = (e >> 1) & 3, h = e & 1;
+    const int src = v == V_W0X ? I::W0X : v == V_W0Y ? I::W0Y : v == V_B0 ? I::B0 : I::G1 + 32 * (v - V_G1);
+    vec[x] = fl[src + 8 * j + 2 * q + h];
+  }
+  for (int x = tid; x < 5 * 4 * 4; x += 128) {  // [layer][tq][j]
+    const int l = x >> 4, q = (x >> 2) & 3, j = x & 3;
+    const float bx = fl[I::BH + 32 * l + 8 * j + 2 * q], by = fl[I::BH + 32 * l + 8 * j + 2 * q + 1];
+    biasq[x] = make_float4(bx, by, bx, by);
+  }
+}
+
+// smallest value above k whose low kIdxBits bits carry the point's index: keys become unique (a REDUX round removes exactly one entry);
+// rounding an upper bound UP only widens the candidate set
+template <int kIdxBits>
+__device__ __forceinline__ uint32_t unique_key(uint32_t k, int idx) {
+  constexpr uint32_t kIdxMask = (1u << kIdxBits) - 1u;
+  return ((min(k, 0xFFFFF000u) + (kIdxMask + 1u)) & ~kIdxMask) | (uint32_t)idx;
+}
+
+// geometry rows of the lane's two head channels 2 tq, 2 tq + 1 (zero beyond E: their partial distance is 0)
+struct HeadGeo {
+  float gx0, gy0, h0, gx1, gy1, h1;
+};
+__device__ __forceinline__ HeadGeo head_geo(const DuneParams& prm, int tq) {
+  const int e0 = 2 * tq, e1 = 2 * tq + 1, E = prm.geo.E;
+  HeadGeo hg;
+  hg.gx0 = e0 < E ? prm.geo.G[e0][0] : 0.f; hg.gy0 = e0 < E ? prm.geo.G[e0][1] : 0.f; hg.h0 = e0 < E ? prm.geo.h[e0] : 0.f;
+  hg.gx1 = e1 < E ? prm.geo.G[e1][0] : 0.f; hg.gy1 = e1 < E ? prm.geo.G[e1][1] : 0.f; hg.h1 = e1 < E ? prm.geo.h[e1] : 0.f;
+  return hg;
+}
+
+// one warp's 32 points through the screening network: (x0, y0) = the lane's own point in the robot frame (zeros for rows beyond n);
+// returns its screened distance d~ and error radius eps.  vq / wl / bqq: the lane's views of the staged operands.
+__device__ __forceinline__ void screen_point(const DuneParams& prm, const HeadGeo& hg, const float* __restrict__ vq, const uint4* __restrict__ wl,
+                                             const float4* __restrict__ bqq, int lane, float x0, float y0, float& d, float& eps) {
+  const int tq = lane & 3;
+  float xr[4], yr[4];
+#pragma unroll
+  for (int r = 0; r < 4; ++r) {
+    xr[r] = __shfl_sync(0xffffffffu, x0, (lane & ~3) | r);
+    yr[r] = __shfl_sync(0xffffffffu, y0, (lane & ~3) | r);
+  }
+  f2 acc[4][4];
+  uint32_t a[2][2][4];
+  {  // layer 0 (2 -> 32) on the FMA pipe, directly in accumulator layout
+    const ulonglong2 wx01 = *reinterpret_cast<const ulonglong2*>(vq + 32 * V_W0X), wx23 = *reinterpret_cast<const ulonglong2*>(vq + 32 * V_W0X + 4);
+    const ulonglong2 wy01 = *reinterpret_cast<const ulonglong2*>(vq + 32 * V_W0Y), wy23 = *reinterpret_cast<const ulonglong2*>(vq + 32 * V_W0Y + 4);
+    const ulonglong2 b01 = *reinterpret_cast<const ulonglong2*>(vq + 32 * V_B0), b23 = *reinterpret_cast<const ulonglong2*>(vq + 32 * V_B0 + 4);
+    const f2 wx[4] = {wx01.x, wx01.y, wx23.x, wx23.y}, wy[4] = {wy01.x, wy01.y, wy23.x, wy23.y}, bb[4] = {b01.x, b01.y, b23.x, b23.y};
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+      const f2 x2 = tc::pk(xr[r], xr[r]), y2 = tc::pk(yr[r], yr[r]);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) acc[r][j] = tc::fma2(wy[j], y2, tc::fma2(wx[j], x2, bb[j]));
+    }
+  }
+  ln_tanh_frag(acc, vq + 32 * V_G1, vq + 32 * V_BE1, lane, a);
+  dense_frag<4>(wl + 0 * 128, bqq + 16 * 0, a, acc);
+  relu_frag(acc, a);
+  dense_frag<4>(wl + 1 * 128, bqq + 16 * 1, a, acc);
+  ln_tanh_frag(acc, vq + 32 * V_G6, vq + 32 * V_BE6, lane, a);
+  dense_frag<4>(wl + 2 * 128, bqq + 16 * 2, a, acc);
+  relu_frag(acc, a);
+  dense_frag<4>(wl + 3 * 128, bqq + 16 * 3, a, acc);
+  ln_tanh_frag(acc, vq + 32 * V_G11, vq + 32 * V_BE11, lane, a);
+  f2 mu[4][1];
+  dense_frag<1>(wl + 4 * 128, bqq + 16 * 4, a, mu);
+
+  // head: d~ = relu(mu)^T (G p0 - h): partial over the lane's two channels for each row slot, transposing quad reduction
+  float dp[4];
+#pragma unroll
+  for (int r = 0; r < 4; ++r) {
+    float m0, m1;
+    tc::upk(mu[r][0], m0, m1);
+    const float ge0 = fmaf(hg.gy0, yr[r], hg.gx0 * xr[r]) - hg.h0, ge1 = fmaf(hg.gy1, yr[r], hg.gx1 * xr[r]) - hg.h1;
+    dp[r] = fmaf(fmaxf(m1, 0.f), ge1, fmaxf(m0, 0.f) * ge0);
+  }
+  d = quad_transpose_sum(dp, tq);  // the lane's own point
+  float sa = 0.f;
+#pragma unroll
+  for (int e = 0; e < kMaxEdges; ++e)
+    if (e < prm.geo.E) sa += fabsf(fmaf(prm.geo.G[e][1], y0, prm.geo.G[e][0] * x0) - prm.geo.h[e]);
+  eps = fmaf(prm.c_mu, sa, 1e-4f);
+}
+
 }  // namespace sm
 
 // shared memory: B fragments | permuted vectors | bias fragments | raw points of the item in flight (x | y | vx | vy, N floats each) |
@@ -171,7 +274,6 @@ __host__ __device__ inline size_t dune_screen_mma_smem_bytes(int N, int M) {
 template <int kP>
 __global__ void __launch_bounds__(128, kP <= 4 ? NB_SMMA_BLOCKS : 4) dune_screen_mma_kernel(const DuneParams prm, const unsigned char* __restrict__ image) {
   extern __shared__ __align__(1024) unsigned char smem_dyn[];
-  using I = TcImage;
   uint4* wfrag = reinterpret_cast<uint4*>(smem_dyn);
   float* vec = reinterpret_cast<float*>(smem_dyn + sm::kFragBytes);
   float4* biasq = reinterpret_cast<float4*>(smem_dyn + sm::kFragBytes + sm::kVecBytes);
@@ -182,45 +284,19 @@ __global__ void __launch_bounds__(128, kP <= 4 ? NB_SMMA_BLOCKS : 4) dune_screen
   __shared__ float ldt_s[kCandMax];
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, tq = lane & 3;
-  // ---- operand staging: the screen image of dune_screen_kernel (K-major UMMA layout, hi halves) re-ordered into mma.sync B fragments
-  {
-    uint32_t* wf = reinterpret_cast<uint32_t*>(wfrag);
-    for (int x = tid; x < sm::kFragBytes / 4; x += 128) {
-      const int c = x & 3, ln = (x >> 2) & 31, jp = (x >> 7) & 1, s = (x >> 8) & 1, l = x >> 9;
-      const int n = 8 * (2 * jp + (c >> 1)) + (ln >> 2), k = 16 * s + 2 * (ln & 3) + 8 * (c & 1);
-      const size_t off = (size_t)l * I::kLayerStride + (size_t)(k / 16) * 1024 + ((k % 16) / 8) * 512 + (n / 8) * 128 + (n % 8) * 16 + (k % 8) * 2;
-      wf[x] = *reinterpret_cast<const uint32_t*>(image + off);
-    }
-    const float* fl = reinterpret_cast<const float*>(image + I::kFloatOff);
-    for (int x = tid; x < sm::kVecs * 32; x += 128) {
-      const int v = x >> 5, e = x & 31, q = e >> 3, j = (e >> 1) & 3, h = e & 1;
-      const int src = v == sm::V_W0X ? I::W0X : v == sm::V_W0Y ? I::W0Y : v == sm::V_B0 ? I::B0 : I::G1 + 32 * (v - sm::V_G1);
-      vec[x] = fl[src + 8 * j + 2 * q + h];
-    }
-    for (int x = tid; x < 5 * 4 * 4; x += 128) {  // [layer][tq][j]
-      const int l = x >> 4, q = (x >> 2) & 3, j = x & 3;
-      const float bx = fl[I::BH + 32 * l + 8 * j + 2 * q], by = fl[I::BH + 32 * l + 8 * j + 2 * q + 1];
-      biasq[x] = make_float4(bx, by, bx, by);
-    }
-    if (tid < 2) cnt_s[tid] = 0;
-  }
+  sm::stage_operands(image, smem_dyn, tid);
+  if (tid < 2) cnt_s[tid] = 0;
   __syncthreads();
   const uint4* wl = wfrag + lane;
   const float* vq = vec + 8 * tq;
   const float4* bqq = biasq + 4 * tq;
 
-  const int T1 = prm.T + 1, N = prm.N, M = prm.M, E = prm.geo.E;
+  const int T1 = prm.T + 1, N = prm.N, M = prm.M;
   const int items = prm.B * T1;
-  // geometry rows of this lane's two head channels (zero beyond E: their partial distance is 0)
-  const int e0 = 2 * tq, e1 = 2 * tq + 1;
-  const float gx0 = e0 < E ? prm.geo.G[e0][0] : 0.f, gy0 = e0 < E ? prm.geo.G[e0][1] : 0.f, h0 = e0 < E ? prm.geo.h[e0] : 0.f;
-  const float gx1 = e1 < E ? prm.geo.G[e1][0] : 0.f, gy1 = e1 < E ? prm.geo.G[e1][1] : 0.f, h1 = e1 < E ? prm.geo.h[e1] : 0.f;
+  const sm::HeadGeo hg = sm::head_geo(prm, tq);
   const int own0 = 32 * warp + 8 * tq + g;  // the lane's point in pass 0 (pass p: + 128 p)
   constexpr int kIdxBits = kP <= 4 ? 9 : 10;
   constexpr uint32_t kIdxMask = (1u << kIdxBits) - 1u;
-  // smallest value above k whose low kIdxBits bits carry the point's index: keys become unique (a REDUX round removes exactly one entry);
-  // rounding an upper bound UP only widens the candidate set
-  auto unique_key = [&](uint32_t k, int idx) -> uint32_t { return ((min(k, 0xFFFFF000u) + (kIdxMask + 1u)) & ~kIdxMask) | (uint32_t)idx; };
 
   // The raw point data of an item are copied asynchronously (cp.async, each thread exactly the <= 4 entries it reads itself: no
   // barrier) -- for the NEXT item as soon as this thread has read its last point of the current one.
@@ -301,56 +377,11 @@ __global__ void __launch_bounds__(128, kP <= 4 ? NB_SMMA_BLOCKS : 4) dune_screen
         x0 = fmaf(fr.cs, dx, fr.sn * dy);
         y0 = fmaf(fr.cs, dy, -(fr.sn * dx));
       }
-      float xr[4], yr[4];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        xr[r] = __shfl_sync(0xffffffffu, x0, (lane & ~3) | r);
-        yr[r] = __shfl_sync(0xffffffffu, y0, (lane & ~3) | r);
-      }
-      sm::f2 acc[4][4];
-      uint32_t a[2][2][4];
-      {  // layer 0 (2 -> 32) on the FMA pipe, directly in accumulator layout
-        const ulonglong2 wx01 = *reinterpret_cast<const ulonglong2*>(vq + 32 * sm::V_W0X), wx23 = *reinterpret_cast<const ulonglong2*>(vq + 32 * sm::V_W0X + 4);
-        const ulonglong2 wy01 = *reinterpret_cast<const ulonglong2*>(vq + 32 * sm::V_W0Y), wy23 = *reinterpret_cast<const ulonglong2*>(vq + 32 * sm::V_W0Y + 4);
-        const ulonglong2 b01 = *reinterpret_cast<const ulonglong2*>(vq + 32 * sm::V_B0), b23 = *reinterpret_cast<const ulonglong2*>(vq + 32 * sm::V_B0 + 4);
-        const sm::f2 wx[4] = {wx01.x, wx01.y, wx23.x, wx23.y}, wy[4] = {wy01.x, wy01.y, wy23.x, wy23.y}, bb[4] = {b01.x, b01.y, b23.x, b23.y};
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-          const sm::f2 x2 = tc::pk(xr[r], xr[r]), y2 = tc::pk(yr[r], yr[r]);
-#pragma unroll
-          for (int j = 0; j < 4; ++j) acc[r][j] = tc::fma2(wy[j], y2, tc::fma2(wx[j], x2, bb[j]));
-        }
-      }
-      sm::ln_tanh_frag(acc, vq + 32 * sm::V_G1, vq + 32 * sm::V_BE1, lane, a);
-      sm::dense_frag<4>(wl + 0 * 128, bqq + 16 * 0, a, acc);
-      sm::relu_frag(acc, a);
-      sm::dense_frag<4>(wl + 1 * 128, bqq + 16 * 1, a, acc);
-      sm::ln_tanh_frag(acc, vq + 32 * sm::V_G6, vq + 32 * sm::V_BE6, lane, a);
-      sm::dense_frag<4>(wl + 2 * 128, bqq + 16 * 2, a, acc);
-      sm::relu_frag(acc, a);
-      sm::dense_frag<4>(wl + 3 * 128, bqq + 16 * 3, a, acc);
-      sm::ln_tanh_frag(acc, vq + 32 * sm::V_G11, vq + 32 * sm::V_BE11, lane, a);
-      sm::f2 mu[4][1];
-      sm::dense_frag<1>(wl + 4 * 128, bqq + 16 * 4, a, mu);
-
-      // head: d~ = relu(mu)^T (G p0 - h): partial over the lane's two channels for each row slot, transposing quad reduction
-      float dp[4];
-#pragma unroll
-      for (int r = 0; r < 4; ++r) {
-        float m0, m1;
-        tc::upk(mu[r][0], m0, m1);
-        const float ge0 = fmaf(gy0, yr[r], gx0 * xr[r]) - h0, ge1 = fmaf(gy1, yr[r], gx1 * xr[r]) - h1;
-        dp[r] = fmaf(fmaxf(m1, 0.f), ge1, fmaxf(m0, 0.f) * ge0);
-      }
-      const float d = sm::quad_transpose_sum(dp, tq);  // the lane's own point
-      float sa = 0.f;
-#pragma unroll
-      for (int e = 0; e < kMaxEdges; ++e)
-        if (e < E) sa += fabsf(fmaf(prm.geo.G[e][1], y0, prm.geo.G[e][0] * x0) - prm.geo.h[e]);
-      const float eps = fmaf(prm.c_mu, sa, 1e-4f);
+      float d, eps;
+      sm::screen_point(prm, hg, vq, wl, bqq, lane, x0, y0, d, eps);
 #pragma unroll
       for (int j = kP - 1; j > 0; --j) { kk[j] = kk[j - 1]; ll[j] = ll[j - 1]; dd[j] = dd[j - 1]; }
-      kk[0] = i < n ? unique_key(orderable(d + eps), i) : 0xFFFFFFFFu;
+      kk[0] = i < n ? sm::unique_key<kIdxBits>(orderable(d + eps), i) : 0xFFFFFFFFu;
       ll[0] = d - eps; dd[0] = d;
     }
     if (item + (int)gridDim.x < items) {  // this thread is done with `raw`: its part of the next item
@@ -424,6 +455,169 @@ __global__ void __launch_bounds__(128, kP <= 4 ? NB_SMMA_BLOCKS : 4) dune_screen
     par ^= 1;
   }
   tc::cp_async_wait_all();
+}
+
+
+// ---- The default shape: one warp per (environment, step) item.
+//
+// dune_screen_mma_kernel above spreads an item over the 4 warps of a CTA, and every warp pays an item skeleton of its own: the
+// accurate cos / sin of the item frame, cp.async staging, M REDUX rounds over its keys and M more to merge the 4 M survivors, a
+// shared-memory candidate counter and two block barriers -- 856 of the 3,852 instructions a warp spends on an item at N = 500.  Here
+// one warp takes an item from its frame to its candidate list and shares nothing with the other warps but the staged operands:
+//  * per 32-point tile: the same network, keys and bounds (sm::screen_point, sm::unique_key), hence the same tau and the same
+//    candidate set; only the order of the list differs (the refine kernel ranks candidates by (distance, index));
+//  * points: the lane's point of the NEXT tile is loaded into registers while the current tile runs (plain loads: the T + 1 items of
+//    an environment read the same points, mostly from L2);
+//  * d~ and eps of the lane's point of every tile go to the warp's slab in shared memory, written and read by that lane only (no
+//    barrier); after the last tile the network's registers are free, the <= 4 kP keys of the lane are rebuilt there and M REDUX rounds
+//    over them give tau -- no merge;
+//  * the candidate list is compacted with __ballot_sync and a __popc prefix and written straight to global memory;
+//  * items are handed out by a counter (flag_count[3], zeroed by the launcher with the other three words), the next ticket requested
+//    while the current item runs: at ~7 items per warp and launch a static stride leaves a tail of up to one item.
+// The only block barrier is the one after the operand staging.
+
+// shared memory: B fragments | permuted vectors | bias fragments | per warp: d~ and eps of its item (N rounded up to 32, 4 B each)
+__host__ __device__ inline size_t dune_screen_warp_smem_bytes(int N) {
+  return (size_t)sm::kFragBytes + sm::kVecBytes + sm::kBiasQBytes + (size_t)4 * 2 * ((N + 31) / 32 * 32) * 4;
+}
+
+// kP: as above (N <= 128 kP): the lane rebuilds its <= 4 kP keys in registers for the selection
+template <int kP>
+__global__ void __launch_bounds__(128, kP <= 4 ? NB_SMMA_BLOCKS : 4) dune_screen_warp_kernel(const DuneParams prm, const unsigned char* __restrict__ image) {
+  extern __shared__ __align__(1024) unsigned char smem_dyn[];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, tq = lane & 3;
+  const int T1 = prm.T + 1, N = prm.N, M = prm.M;
+  sm::stage_operands(image, smem_dyn, tid);
+  if (prm.skip_t0)  // step-0 items are not handed out below: same inputs as in the previous PAN iteration, its outputs stand
+    for (int b = blockIdx.x * 128 + tid; b < prm.B; b += gridDim.x * 128) prm.cand_cnt[(size_t)b * T1] = 0;
+  __syncthreads();
+  const uint4* wl = reinterpret_cast<const uint4*>(smem_dyn) + lane;
+  const float* vq = reinterpret_cast<const float*>(smem_dyn + sm::kFragBytes) + 8 * tq;
+  const float4* bqq = reinterpret_cast<const float4*>(smem_dyn + sm::kFragBytes + sm::kVecBytes) + 4 * tq;
+  const int np = (N + 31) & ~31;
+  float* sd = reinterpret_cast<float*>(smem_dyn + sm::kFragBytes + sm::kVecBytes + sm::kBiasQBytes) + (size_t)warp * 2 * np;  // [tile][lane]
+  float* se = sd + np;
+  const sm::HeadGeo hg = sm::head_geo(prm, tq);
+  const int own = 8 * tq + (lane >> 2);  // the lane's point in a tile
+  constexpr int kIdxBits = kP <= 4 ? 9 : 10;
+  constexpr int kTiles = 4 * kP;
+  const unsigned lanes_below = (1u << lane) - 1u;
+
+  auto run_item = [&](int b, int t) {
+    const int item = b * T1 + t;
+    int32_t* out_idx = prm.cand_idx + (size_t)item * kCandMax;
+    float* out_dt = prm.cand_dt + (size_t)item * kCandMax;
+    const int act = prm.active ? prm.active[b] : 1;
+    if (act == 0) {
+      if (lane == 0) prm.cand_cnt[item] = 0;
+      return;
+    }
+    int n = prm.num_points ? prm.num_points[b] : N;
+    n = n < 0 ? 0 : (n > N ? N : n);
+    if (t == 0 && lane == 0) {
+      prm.sel_count[b] = n < M ? n : M;
+      if (n == 0 && prm.min_dist) prm.min_dist[b] = __int_as_float(0x7f800000);
+    }
+    if (n <= kCandMax && !prm.calibrate) {  // nothing to screen: every point is a candidate
+      if (lane < n) { out_idx[lane] = lane; out_dt[lane] = __int_as_float(0x7fc00000); }
+      if (lane == 0) { prm.cand_cnt[item] = n; tc::refine_append(prm, item, n); }
+      return;
+    }
+    const tc::ItemFrame fr = tc::item_frame(prm, b, t);
+    const int tiles = (n + 31) >> 5;
+    float px = 0.f, py = 0.f, pvx = 0.f, pvy = 0.f;  // the lane's point of the next tile
+    auto fetch = [&](int i) {
+      if (i < n) {
+        px = fr.px[i]; py = fr.py[i];
+        if (fr.vx) { pvx = fr.vx[i]; pvy = fr.vy[i]; }
+      }
+    };
+    fetch(own);
+#pragma unroll 1
+    for (int tile = 0; tile < tiles; ++tile) {
+      const int i = 32 * tile + own;
+      float gx = px, gy = py;
+      const float vx = pvx, vy = pvy;
+      fetch(i + 32);
+      float x0 = 0.f, y0 = 0.f;
+      if (i < n) {  // rows beyond n run on zeros (their results are never looked at)
+        if (fr.vx) {
+          gx = flow(gx, vx, fr.dt, fr.t);
+          gy = flow(gy, vy, fr.dt, fr.t);
+        }
+        const float dx = gx - fr.sx, dy = gy - fr.sy;
+        x0 = fmaf(fr.cs, dx, fr.sn * dy);
+        y0 = fmaf(fr.cs, dy, -(fr.sn * dx));
+      }
+      float d, eps;
+      sm::screen_point(prm, hg, vq, wl, bqq, lane, x0, y0, d, eps);
+      sd[32 * tile + lane] = d;
+      se[32 * tile + lane] = eps;
+    }
+    if (n <= kCandMax) {  // calibration mode: all points (one tile), with their screened distance
+      if (own < n) { out_idx[own] = own; out_dt[own] = sd[lane]; }
+      if (lane == 0) { prm.cand_cnt[item] = n; tc::refine_append(prm, item, n); }
+      return;
+    }
+    // tau = the M-th smallest upper bound: the keys are unique, so each REDUX round removes exactly one of them (n > kCandMax >= M:
+    // M finite keys exist)
+    uint32_t q[kTiles];
+#pragma unroll
+    for (int j = 0; j < kTiles; ++j) {
+      const int i = 32 * j + own;
+      q[j] = i < n ? sm::unique_key<kIdxBits>(orderable(sd[32 * j + lane] + se[32 * j + lane]), i) : 0xFFFFFFFFu;
+    }
+    uint32_t tau;
+    for (int m = 0;; ++m) {
+      uint32_t mine = q[0];
+#pragma unroll
+      for (int j = 1; j < kTiles; ++j) mine = min(mine, q[j]);
+      tau = __reduce_min_sync(0xffffffffu, mine);
+      if (m == M - 1) break;
+#pragma unroll
+      for (int j = 0; j < kTiles; ++j) q[j] = q[j] == tau ? 0xFFFFFFFFu : q[j];
+    }
+    // candidates: lower bound <= tau, in (tile, lane) order
+    int nc = 0;
+#pragma unroll
+    for (int j = 0; j < kTiles; ++j) {
+      if (32 * j < n) {  // warp-uniform
+        const int i = 32 * j + own;
+        const float d = sd[32 * j + lane];
+        const bool take = i < n && orderable(d - se[32 * j + lane]) <= tau;
+        const unsigned bal = __ballot_sync(0xffffffffu, take);
+        const int pos = nc + __popc(bal & lanes_below);
+        if (take && pos < kCandMax) { out_idx[pos] = i; out_dt[pos] = d; }
+        nc += __popc(bal);
+      }
+    }
+    if (lane == 0) {
+      if (nc <= kCandMax) {
+        prm.cand_cnt[item] = nc;
+        tc::refine_append(prm, item, nc);
+        atomicAdd(&prm.screen_stats[2], (unsigned)nc);
+        atomicAdd(&prm.screen_stats[3], 1u);
+      } else {
+        prm.cand_cnt[item] = -1;  // too many candidates: the exact kernel evaluates this item in full
+        atomicAdd(&prm.screen_stats[1], 1u);
+        prm.flag_list[atomicAdd(prm.flag_count, 1)] = item;
+      }
+    }
+  };
+
+  const int steps = prm.skip_t0 ? prm.T : T1;  // items handed out per environment (t = 1..T with skip_t0)
+  const int work = prm.B * steps;
+  int* const counter = prm.flag_count + 3;
+  int w = 0;
+  if (lane == 0) w = atomicAdd(counter, 1);
+  w = __shfl_sync(0xffffffffu, w, 0);
+  while (w < work) {
+    int next = 0;
+    if (lane == 0) next = atomicAdd(counter, 1);
+    const int b = w / steps;
+    run_item(b, w - b * steps + (prm.skip_t0 ? 1 : 0));
+    w = __shfl_sync(0xffffffffu, next, 0);
+  }
 }
 
 }  // namespace nb

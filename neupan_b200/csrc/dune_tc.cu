@@ -138,11 +138,15 @@ int launch_dune_tc(const DuneParams& prm_in, const unsigned char* d_image, const
     int per_s = (int)(233472 / (smem_s + 2048));
     per_s = per_s > 4 ? 4 : (per_s < 1 ? 1 : per_s);
     const int screen_mma = prm.screen_mma;
-    cudaError_t e = cudaMemsetAsync(prm.flag_count, 0, 3 * sizeof(int32_t), st);
-    const size_t smem_m = dune_screen_mma_smem_bytes(prm.N, prm.M);
+    cudaError_t e = cudaMemsetAsync(prm.flag_count, 0, 4 * sizeof(int32_t), st);
+    // one warp per item where the launch has at least one item per resident warp; smaller batches keep the 4 warps of a CTA on one item
+    // (an item's tiles would otherwise run one after another on a single warp while most warp slots idle).  2 / 3 force the CTA / warp shape.
+    const int warp_slots = sm_count * (prm.N <= 512 ? NB_SMMA_BLOCKS : 4) * 4;
+    const bool per_warp = screen_mma == 3 || (screen_mma != 2 && items_ >= warp_slots);
+    const size_t smem_m = per_warp ? dune_screen_warp_smem_bytes(prm.N) : dune_screen_mma_smem_bytes(prm.N, prm.M);
     if (screen_mma && prm.N <= 1024 && (long long)smem_m <= max_smem_optin) {  // larger clouds: the tcgen05 screen kernel (key arrays in shared memory)
-      // no TMEM in this kernel: residency is whatever registers and shared memory admit
-      auto go = [&](auto kern, int& per_m, size_t& per_m_smem) {
+      // no TMEM in these kernels: residency is whatever registers and shared memory admit
+      auto go = [&](auto kern, int& per_m, size_t& per_m_smem, int work) {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_m);
         if (e == cudaSuccess && (per_m < 0 || per_m_smem != smem_m)) {
           e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_m, kern, 128, smem_m);
@@ -156,15 +160,18 @@ int launch_dune_tc(const DuneParams& prm_in, const unsigned char* d_image, const
             cap = v ? atoi(v) : 0;
           }
           int grid = sm_count * ((cap > 0 && cap < per_m) ? cap : per_m);
-          if (grid > items_) grid = items_;
+          if (grid > work) grid = work;
           kern<<<grid, 128, smem_m, st>>>(prm, d_screen_image);
           e = cudaGetLastError();
         }
       };
-      static int per4 = -1, per8 = -1;
-      static size_t smem4 = 0, smem8 = 0;
-      if (prm.N <= 512) go(dune_screen_mma_kernel<4>, per4, smem4);
-      else go(dune_screen_mma_kernel<8>, per8, smem8);
+      static int per4 = -1, per8 = -1, perw4 = -1, perw8 = -1;
+      static size_t smem4 = 0, smem8 = 0, smemw4 = 0, smemw8 = 0;
+      const int warp_ctas = (items_ + 3) / 4;  // one item per warp at a time
+      if (per_warp && prm.N <= 512) go(dune_screen_warp_kernel<4>, perw4, smemw4, warp_ctas);
+      else if (per_warp) go(dune_screen_warp_kernel<8>, perw8, smemw8, warp_ctas);
+      else if (prm.N <= 512) go(dune_screen_mma_kernel<4>, per4, smem4, items_);
+      else go(dune_screen_mma_kernel<8>, per8, smem8, items_);
     } else {
       if (e == cudaSuccess) e = cudaFuncSetAttribute(dune_screen_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_s);
       if (e == cudaSuccess) {

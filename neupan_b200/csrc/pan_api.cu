@@ -117,6 +117,7 @@ struct nb_pan {
   int* work_counters = nullptr;     // dynamic env -> warp assignment of the NRMP kernel, one counter per internal stream
   int dune_skip_t0 = 1;             // NB_OPT_DUNE_SKIP_T0: PAN iterations k > 0 keep the step-0 items of iteration 0 (screening variant)
   int screen_mma = 1;               // NB_OPT_DUNE_SCREEN_MMA: screening pass on mma.sync (N <= 512) instead of tcgen05
+  int screen_shape = 1;             // the mma.sync screening pass: 1 = by batch size, 2 = one CTA of 4 warps per item, 3 = one warp per item (NB_SCREEN_MMA)
   int nrmp_defer_stop_min = 256;    // NB_NRMP_DEFER_STOP_MIN (developer switch, read at create): smallest batch whose stop criterion runs as its own kernel
   int nrmp_dynamic = 1;             // NB_NRMP_STATIC=1 (developer switch, read at create) turns the persistent-warp schedule off
   float* warm = nullptr;            // NRMP warm-start records, nrmp_warm_floats(T, M) per environment
@@ -306,7 +307,7 @@ int calibrate_screen(nb_pan* p, cudaStream_t st) {
     prm.cand_idx = p->cand_idx; prm.cand_cnt = p->cand_cnt; prm.cand_dt = p->cand_dt; prm.screen_stats = p->screen_stats; prm.c_mu = p->c_mu;
     prm.flag_list = p->flag_list; prm.flag_count = p->flag_count; prm.refine_list = p->refine_list; prm.calibrate = 1;
     for (int shape = 0; shape < 2 && rc == NB_OK; ++shape) {  // both screening kernels (tcgen05 / mma.sync): the bound holds whichever option is set later
-      prm.screen_mma = shape;
+      prm.screen_mma = shape ? p->screen_shape : 0;
       rc = launch_dune(p, prm, st);
       if (rc == NB_OK && cudaStreamSynchronize(st) != cudaSuccess) rc = fail(NB_ERR_CUDA, "calibrate_screen: kernel failed");
     }
@@ -409,7 +410,7 @@ int nb_pan_create(const nb_pan_config* cfg, const float* weights, int64_t n_weig
     NB_CUDA(dalloc(&p->cand_dt, (size_t)cfg->max_envs * (cfg->receding + 1) * nb::kCandMax));
     NB_CUDA(dalloc(&p->cand_cnt, (size_t)cfg->max_envs * (cfg->receding + 1)));
     NB_CUDA(dalloc(&p->flag_list, (size_t)cfg->max_envs * (cfg->receding + 1)));
-    NB_CUDA(dalloc(&p->flag_count, (size_t)32));  // 4 words per internal stream: flagged items, the two refine list lengths
+    NB_CUDA(dalloc(&p->flag_count, (size_t)32));  // 4 words per internal stream: flagged items, the two refine list lengths, the screen item counter
     NB_CUDA(dalloc(&p->refine_list, (size_t)2 * cfg->max_envs * (cfg->receding + 1)));
     NB_CUDA(dalloc(&p->screen_stats, (size_t)4));
     NB_CUDA(cudaMemset(p->screen_stats, 0, 4 * sizeof(unsigned)));
@@ -439,7 +440,10 @@ int nb_pan_create(const nb_pan_config* cfg, const float* weights, int64_t n_weig
   if (const char* e = getenv("NB_NRMP_DEFER_STOP_MIN")) p->nrmp_defer_stop_min = atoi(e);
   if (const char* e = getenv("NB_H2D_CHUNKS")) { p->h2d_chunks = atoi(e); if (p->h2d_chunks < 1) p->h2d_chunks = 1; if (p->h2d_chunks > nb_pan::kMaxChunks) p->h2d_chunks = nb_pan::kMaxChunks; }
   if (const char* e = getenv("NB_DUNE_SKIP_T0")) p->dune_skip_t0 = atoi(e) != 0;  // developer overrides of the option defaults
-  if (const char* e = getenv("NB_SCREEN_MMA")) p->screen_mma = atoi(e) != 0;
+  if (const char* e = getenv("NB_SCREEN_MMA")) {  // 0 / 1: the option's initial value; 2 / 3: on, with the CTA-per-item / warp-per-item kernel
+    p->screen_mma = atoi(e) != 0;
+    p->screen_shape = atoi(e) == 2 || atoi(e) == 3 ? atoi(e) : 1;
+  }
   if (const char* e = getenv("NB_NRMP_RESTART_IT")) p->warm_check_it = atoi(e);
   if (const char* e = getenv("NB_NRMP_RESTART_GAP")) p->warm_check_gap = atof(e);
   NB_CUDA(cudaMemset(p->warm_valid, 0, B * sizeof(int32_t)));
@@ -558,7 +562,7 @@ int nb_dune_forward(nb_pan_t* p, int32_t B, int32_t N, const float* nom_s, const
   prm.min_dist = out_min_distance;
   prm.B = B; prm.N = N; prm.T = p->cfg.receding; prm.M = p->cfg.nrmp_max_num; prm.dt = (float)p->cfg.step_time; prm.geo = p->geo;
   prm.cand_idx = p->cand_idx; prm.cand_cnt = p->cand_cnt; prm.cand_dt = p->cand_dt; prm.screen_stats = p->screen_stats; prm.c_mu = p->c_mu;
-  prm.flag_list = p->flag_list; prm.flag_count = p->flag_count; prm.refine_list = p->refine_list; prm.screen_mma = p->screen_mma;
+  prm.flag_list = p->flag_list; prm.flag_count = p->flag_count; prm.refine_list = p->refine_list; prm.screen_mma = p->screen_mma ? p->screen_shape : 0;
   return launch_dune(p, prm, (cudaStream_t)stream);
 }
 
@@ -647,7 +651,7 @@ int pan_forward_impl(nb_pan_t* p, int32_t B, int32_t N, const float* nom_s, cons
         d.cand_idx = p->cand_idx + (size_t)lo * T1s * nb::kCandMax; d.cand_dt = p->cand_dt + (size_t)lo * T1s * nb::kCandMax;
         d.cand_cnt = p->cand_cnt + (size_t)lo * T1s; d.screen_stats = p->screen_stats; d.c_mu = p->c_mu;
         d.flag_list = p->flag_list + (size_t)lo * T1s; d.flag_count = p->flag_count + 4 * counter_slot; d.refine_list = p->refine_list + (size_t)2 * lo * T1s;
-        d.screen_mma = p->screen_mma;
+        d.screen_mma = p->screen_mma ? p->screen_shape : 0;
         d.skip_t0 = (k > 0 && p->dune_skip_t0) ? 1 : 0;  // the step-0 items of iteration 0 stand (DuneParams::skip_t0)
         if (k == 0 && plan && plan->n > 1) {
           // the first DUNE pass of this range chunk by chunk, each as soon as its points have landed: the upload of chunk c+1 overlaps the
